@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the COVINS hot path on B200 (contract: see DESIGN.md §Measurement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--gba-config C3]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--gba-config C3] [--dump-outputs DIR]
 
 Metric (BASELINE.json): global-BA iterations/s & descriptor-match Gpairs/s on the 5-agent EuRoC-sized synthetic map
 (config C3: 2000 KF / 100k LM / ~800k obs; 1000 ORB features per KF).  One "step" is one pass of the hot path: one outer
@@ -121,6 +121,27 @@ class ClockSampler:
 
 def dist_info():
     return int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("LOCAL_RANK", "0"))
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """Writes each array (numpy or torch) as d/<name>.npy so that two builds can be compared output for output:
+    float64 stays float64, every other type becomes float32 (integers up to 2^24 exactly, larger ones float64)."""
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        if a.dtype != np.float64:
+            exact32 = a.dtype.kind == "f" or a.size == 0 or np.abs(a).max() < 2 ** 24
+            a = a.astype(np.float32 if exact32 else np.float64)
+        out[name] = a
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"outputs take {total} bytes, more than the {DUMP_LIMIT_BYTES} a dump may hold")
+    os.makedirs(d, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 def _cores():
@@ -381,7 +402,7 @@ def run_ours(args):
     dev_ms = sum(tm[k] for k in ("linearize_ms", "build_schur_ms", "factor_ms", "solve_ms", "step_ms"))
 
     # e2e GBA: the host-buffer C-ABI call a user makes (flatten → H2D → symbolic → iterations → D2H)
-    e2e_iters = max(3, min(args.steps, 10))
+    e2e_iters = args.steps
     e2e_runs = []
     for rep in range(4):   # the whole call (create → iterate → read back) is repeated: one untimed warm-up call (first-use costs
         barrier()          # of the allocator / IPC mappings), then three timed ones of which the median is reported
@@ -419,7 +440,7 @@ def run_ours(args):
                 if done_ < n:
                     ps.restart()
             return done_
-        pgo_steps = max(args.steps, 10)
+        pgo_steps = args.steps
         pgo_iters(args.warmup); ps.restart()
         ctx.sync(); lp = ctx.launch_count(); t0 = time.perf_counter()
         pgo_iters(pgo_steps)
@@ -473,7 +494,7 @@ def run_ours(args):
     def step_match_raw(i):      # raw-pointer API: packed rows only, the operand tiles are expanded inside every call
         return M.match_candidates_hamming(ctx, q, maps[i % N_COPIES], (d_seg, h_seg), THR, RATIO)
 
-    m_steps = max(args.steps, 10)
+    m_steps = args.steps
     for i in range(args.warmup):
         step_match(i)
     barrier()
@@ -499,7 +520,7 @@ def run_ours(args):
     ms_raw = e0.elapsed_time(e1) / 10
 
     h_q = q.cpu().pin_memory().numpy()
-    e2e_steps = 6
+    e2e_steps = args.steps
     for i in range(2):
         M.match_candidates_hamming(ctx, h_q, h_maps_np[i % 2], h_seg, THR, RATIO)
     barrier()
@@ -512,7 +533,7 @@ def run_ours(args):
     # e2e through the resident-map API (cvb_db_*): keyframes uploaded once when they join the map (outside the timed
     # region, as in the server's life cycle), per request the query keyframe goes up and the accepted matches come down.
     h_queries = [np.ascontiguousarray(h_maps_np[0][k * N_FEAT:(k + 1) * N_FEAT]) for k in (123, 777, 1500, 42)]
-    db_steps = max(args.steps, 30)
+    db_steps = args.steps
     d2h_db = 0
     for i in range(3):
         dbs[i % N_COPIES].match_hamming(h_queries[i % 4], THR, RATIO)
@@ -678,6 +699,13 @@ def run_ours(args):
             # bounded sample of the same workload on the host cores (the full same-steps run is `--impl reference`)
             line["cpu_baseline"], _ = cpu_gba(args.gba_config, 4)
             line["match"]["cpu_baseline"] = cpu_match_port()
+        if args.dump_outputs:
+            # the result of the last timed step of each leg, as its caller receives it
+            dump_outputs(args.dump_outputs, {
+                "gba_pose": res["pose"], "gba_speedbias": res["speedbias"], "gba_landmarks": res["lm"],
+                "gba_landmark_owner": res["lm_owner"], "gba_cost_history": res["cost"],
+                "pgo_pose": rp["pose"], "pgo_cost_history": rp["cost"],
+                "match_train": out_m[0], "match_dist": out_m[1], "match_count": out_m[2]})
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -691,7 +719,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--gba-config", default=os.environ.get("COVINS_GBA_CONFIG", "C3"))
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step of each leg computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "ours":
         args.warmup = max(args.warmup, 3)
     if args.impl == "reference":

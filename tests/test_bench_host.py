@@ -60,3 +60,19 @@ def test_dist_info_reads_torchrun_environment(monkeypatch):
     for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK"):
         monkeypatch.delenv(k)
     assert b.dist_info() == (0, 1, 0)
+
+
+def test_dump_outputs_writes_float_arrays_within_the_limit(tmp_path):
+    import numpy as np
+    import pytest
+    b = _bench()
+    pose = np.linspace(0, 1, 14).reshape(2, 7)
+    b.dump_outputs(str(tmp_path / "d"), {"pose": pose, "train": np.array([[-1, 999]], np.int32),
+                                         "dist": np.array([0.5], np.float32), "big": np.array([2 ** 30], np.int64)})
+    got = {n: np.load(tmp_path / "d" / f"{n}.npy") for n in ("pose", "train", "dist", "big")}
+    assert got["pose"].dtype == np.float64 and np.array_equal(got["pose"], pose)
+    assert got["train"].dtype == np.float32 and got["train"].tolist() == [[-1.0, 999.0]]
+    assert got["dist"].dtype == np.float32 and got["big"].dtype == np.float64 and got["big"][0] == 2 ** 30
+    with pytest.raises(ValueError):
+        b.dump_outputs(str(tmp_path / "e"), {"x": np.zeros(b.DUMP_LIMIT_BYTES // 4 + 1, np.float32)})
+    assert not (tmp_path / "e").exists()

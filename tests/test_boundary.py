@@ -3,8 +3,8 @@ product package never touches oracle/; without a GPU the product fails loudly in
 import ctypes
 import os
 import re
-
-import pytest
+import subprocess
+import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -53,12 +53,13 @@ def test_product_never_imports_oracle():
 
 
 def test_no_cpu_fallback_without_gpu():
-    import torch
-    import covins_b200
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(covins_b200.CvbError):
-        covins_b200.Context(0)
+    # a child process with every device hidden, so that the check also runs where a GPU is present
+    code = ("import covins_b200\n"
+            "try:\n    covins_b200.Context(0)\nexcept covins_b200.CvbError:\n    raise SystemExit(0)\n"
+            "raise SystemExit('a context was created without a CUDA device')\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=120)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_shard_rows_cuts_on_keyframe_boundaries():
