@@ -16,6 +16,10 @@ struct cvb_buf {
   size_t cap = 0;
 };
 
+enum { WS_Q = 0, WS_T, WS_SEG, WS_OUT0, WS_OUT1, WS_OUT2, WS_PART_I, WS_PART_D, WS_LIST_I, WS_LIST_D, WS_SKIPA,
+       WS_SKIPB, WS_TMP0, WS_TMP1, WS_FLAG, WS_MISC, WS_CHUNK_PS, WS_CHUNK_OFF, WS_GS0, WS_GS1, WS_GS2, WS_GS3, WS_GS4, WS_GS5, WS_XT, WS_XT_TILE,
+       WS_COUNT };
+
 struct cvb_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
@@ -23,23 +27,15 @@ struct cvb_ctx {
   int64_t launches = 0;
   std::string err;
   // grow-only device workspaces (named slots so independent stages never alias)
-  cvb_buf ws[27];
+  cvb_buf ws[WS_COUNT];
   // pinned host staging
   void* h_pin = nullptr;
   size_t h_pin_cap = 0;
   void* ba = nullptr;  // BA state (owned by ba_*.cu)
-  // resident operand tiles of a train set (set by the map database around its matching call, see tc_match.cu): when the
-  // matcher is handed the packed rows `xt_for`, their pre-expanded tiles are at `xt` / `xt_seg_tile`
-  const uint8_t* xt_for = nullptr;
-  const uint8_t* xt = nullptr;
-  const int32_t* xt_seg_tile = nullptr;
   // every extern "C" entry point holds this lock for its duration (cvb_device_guard): a ctx may be shared between host
   // threads — calls on one ctx are serialised, concurrency comes from one ctx per thread
   mutable std::recursive_mutex mtx;
 };
-
-enum { WS_Q = 0, WS_T, WS_SEG, WS_OUT0, WS_OUT1, WS_OUT2, WS_PART_I, WS_PART_D, WS_LIST_I, WS_LIST_D, WS_SKIPA,
-       WS_SKIPB, WS_TMP0, WS_TMP1, WS_FLAG, WS_MISC, WS_CHUNK_PS, WS_CHUNK_OFF, WS_GS0, WS_GS1, WS_GS2, WS_GS3, WS_GS4, WS_GS5, WS_XT, WS_XT_TILE, WS_XT_PROGRESS };
 
 // cudaFuncSetAttribute applies to the CURRENT device: one flag per (call site, device), so that a process that opens contexts
 // on several GPUs raises the dynamic shared-memory limit on each of them
@@ -55,6 +51,13 @@ struct cvb_once_per_device {
 int cvb_fail(cvb_ctx* ctx, int code, const char* fmt, ...);
 void* cvb_ws(cvb_ctx* ctx, int slot, size_t bytes);          // returns nullptr on failure (ctx->err set)
 void* cvb_pinned(cvb_ctx* ctx, size_t bytes);
+
+// cvb_match_hamming_batch_dev without the entry-point guard (the caller holds it), with the train rows' resident operand
+// tiles when there are any (xt / seg_tile as cvb_tc::TcParams; both null: the tensor-core path expands them per call)
+int cvb_match_hamming_tiles_dev(cvb_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, const int32_t* d_seg_ptr,
+                                const int32_t* h_seg_ptr, int n_seg, float thr, float ratio, int32_t* d_match_train,
+                                float* d_match_dist, int32_t* d_n_matches, const uint8_t* xt, const int32_t* seg_tile,
+                                cudaStream_t st);
 
 #define CVB_CUDA(ctx, call)                                                                         \
   do {                                                                                              \

@@ -279,11 +279,8 @@ int cvb_db_match_hamming_dev(cvb_ctx* ctx, cvb_db* db, const uint8_t* d_q, int n
   if (n_seg == 0) return CVB_OK;
   int rc = refresh_seg(ctx, db);
   if (rc) return rc;
-  ctx->xt_for = db->d_rows; ctx->xt = db->d_xt; ctx->xt_seg_tile = db->d_seg_tile;
-  rc = cvb_match_hamming_batch_dev(ctx, d_q, nq, db->d_rows, db->d_seg, db->seg_ptr.data(), n_seg, thr, ratio, d_match_train,
-                                   d_match_dist, d_n_matches, stream);
-  ctx->xt_for = nullptr; ctx->xt = nullptr; ctx->xt_seg_tile = nullptr;
-  return rc;
+  return cvb_match_hamming_tiles_dev(ctx, d_q, nq, db->d_rows, db->d_seg, db->seg_ptr.data(), n_seg, thr, ratio, d_match_train,
+                                     d_match_dist, d_n_matches, db->d_xt, db->d_seg_tile, cvb_stream(ctx, stream));
 }
 
 int cvb_db_match_hamming(cvb_ctx* ctx, cvb_db* db, const uint8_t* q, int nq, float thr, float ratio,
@@ -321,10 +318,8 @@ int cvb_db_match_hamming(cvb_ctx* ctx, cvb_db* db, const uint8_t* q, int nq, flo
   if (!pin) return CVB_ERR_CUDA;
   memcpy(pin, q, (size_t)nq * 32);
   CVB_CUDA(ctx, cudaMemcpyAsync(db->q.p, pin, (size_t)nq * 32, cudaMemcpyHostToDevice, st));
-  ctx->xt_for = db->d_rows; ctx->xt = db->d_xt; ctx->xt_seg_tile = db->d_seg_tile;   // resident operand tiles of these rows
-  rc = cvb_match_hamming_batch_dev(ctx, (const uint8_t*)db->q.p, nq, db->d_rows, db->d_seg, db->seg_ptr.data(), n_seg,
-                                   thr, ratio, (int32_t*)db->mt.p, (float*)db->md.p, (int32_t*)db->nm.p, nullptr);
-  ctx->xt_for = nullptr; ctx->xt = nullptr; ctx->xt_seg_tile = nullptr;
+  rc = cvb_match_hamming_tiles_dev(ctx, (const uint8_t*)db->q.p, nq, db->d_rows, db->d_seg, db->seg_ptr.data(), n_seg, thr,
+                                   ratio, (int32_t*)db->mt.p, (float*)db->md.p, (int32_t*)db->nm.p, db->d_xt, db->d_seg_tile, st);
   if (rc) return rc;
   db_offsets_kernel<<<1, 1024, 0, st>>>((const int32_t*)db->nm.p, n_seg, (int32_t*)db->off.p);
   CVB_CHECK_LAUNCH(ctx);

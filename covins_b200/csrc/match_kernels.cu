@@ -675,11 +675,13 @@ __global__ void shard_merge_kernel(const int32_t* __restrict__ idx_all, const in
     }
 }
 
-// Common implementation of knn / fused-match for both metrics (device pointers).
+// Common implementation of knn / fused-match for both metrics (device pointers).  xt / seg_tile: the resident operand
+// tiles of the Hamming train rows (cvb_tc::TcParams), null when the caller has none.
 template <class M, int QPT_BIG>
 int knn_dev(cvb_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, const int32_t* d_seg_ptr,
             const int32_t* h_seg_ptr, int n_seg, int k, int32_t* d_idx, void* d_dist, bool filter, float thr,
-            float ratio, int32_t* d_match_train, float* d_match_dist, int32_t* d_n_matches, cudaStream_t st) {
+            float ratio, int32_t* d_match_train, float* d_match_dist, int32_t* d_n_matches, cudaStream_t st,
+            const uint8_t* xt = nullptr, const int32_t* seg_tile = nullptr) {
   CVB_REQUIRE(ctx, ctx != nullptr, "null ctx");
   CVB_REQUIRE(ctx, nq >= 0 && k >= 1 && k <= 4, "bad nq/k");
   int max_len = 0;
@@ -693,31 +695,21 @@ int knn_dev(cvb_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, const 
     CVB_CUDA(ctx, cudaMemsetAsync(d_n_matches, 0, sizeof(int32_t) * n_seg, st));
   }
   if (nq == 0) return CVB_OK;
-  if (cvb_tc::profitable(ctx, nq, n_seg, (long)total, max_len)) {   // tensor-core formulation (tc_match.cu), same results
-    cvb_tc::TcParams tp{};
-    tp.q = d_q; tp.nq = nq; tp.t = d_t; tp.seg_ptr = d_seg_ptr; tp.n_seg = n_seg;
-    tp.out_idx = d_idx; tp.out_dist = d_dist; tp.filter = filter ? 1 : 0; tp.thr = thr; tp.ratio = ratio;
-    tp.match_train = d_match_train; tp.match_dist = d_match_dist; tp.n_matches = d_n_matches;
-    tp.h_seg = h_seg_ptr;
-    if (ctx->xt_for == d_t && ctx->xt) { tp.xt = ctx->xt; tp.seg_tile = ctx->xt_seg_tile; }
-    return cvb_tc::launch(ctx, tp, M::kIsL2 ? 1 : 0, k, st);
-  }
-  {
-    // One very long segment (map-wide k-NN): too few segments to spread over the SMs as they are → cut it into uniform
-    // chunks, run the tensor-core kernel on the chunks and merge the chunk lists exactly (the same (distance, index)
-    // merge that combines GPU shards).
-    const char* e = getenv("COVINS_B200_MATCH_KERNEL");
-    const int nqb = (nq + 127) / 128;
-    const int parts = ctx->sm_count / nqb > 0 ? ctx->sm_count / nqb : 1;
-    if (!filter && n_seg == 1 && !(e && !strcmp(e, "popc")) && (long)nq * total >= (1L << 26) &&
-        total >= (int64_t)parts * 4 * 1024) {
-      int n_ps = parts * 4;
-      int64_t chunk = ((total + n_ps - 1) / n_ps + 127) / 128 * 128;
-      // the tensor-core kernel packs (distance, local index) keys: a chunk must stay below its index range (cvb_tc::profitable
-      // enforces the same bound on ordinary segments)
-      const int64_t max_chunk = ((int64_t)1 << cvb_tc::kIdxBits) - 128;
-      if (chunk > max_chunk) chunk = max_chunk;
-      n_ps = (int)((total + chunk - 1) / chunk);
+  const cvb_tc::Formulation f = cvb_tc::choose(ctx, nq, n_seg, total, max_len, filter);
+  switch (f.kind) {
+    case cvb_tc::Formulation::kPerSegment: {   // tensor-core formulation (tc_match.cu), same results
+      cvb_tc::TcParams tp{};
+      tp.q = d_q; tp.nq = nq; tp.t = d_t; tp.seg_ptr = d_seg_ptr; tp.n_seg = n_seg;
+      tp.out_idx = d_idx; tp.out_dist = d_dist; tp.filter = filter ? 1 : 0; tp.thr = thr; tp.ratio = ratio;
+      tp.match_train = d_match_train; tp.match_dist = d_match_dist; tp.n_matches = d_n_matches;
+      tp.h_seg = h_seg_ptr; tp.xt = xt; tp.seg_tile = seg_tile;
+      return cvb_tc::launch(ctx, tp, M::kIsL2 ? 1 : 0, k, st);
+    }
+    case cvb_tc::Formulation::kChunked: {
+      // One very long segment (map-wide k-NN): cut into uniform chunks, the tensor-core kernel on the chunks and an exact
+      // merge of the chunk lists (the same (distance, index) merge that combines GPU shards).
+      const int64_t chunk = f.chunk;
+      const int n_ps = (int)((total + chunk - 1) / chunk);
       std::vector<int32_t> h_ps((size_t)n_ps + 1), h_off((size_t)n_ps);
       for (int c = 0; c <= n_ps; c++) h_ps[c] = (int32_t)std::min<int64_t>((int64_t)c * chunk, total);
       for (int c = 0; c < n_ps; c++) h_off[c] = (int32_t)((int64_t)c * chunk);
@@ -746,6 +738,8 @@ int knn_dev(cvb_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, const 
       CVB_CHECK_LAUNCH(ctx);
       return CVB_OK;
     }
+    case cvb_tc::Formulation::kScalar:
+      break;
   }
   const Plan pl = make_plan<M>(nq, n_seg, max_len, ctx->sm_count, QPT_BIG, true);
   ScanParams sp{};
@@ -901,6 +895,14 @@ __global__ void __launch_bounds__(128) lm_descriptor_kernel(const uint8_t* __res
   if (lane < 8) reinterpret_cast<uint32_t*>(out_desc + (size_t)l * 32)[lane] = __ldg(reinterpret_cast<const uint32_t*>(D + (size_t)best * 32) + lane);
 }
 
+int cvb_match_hamming_tiles_dev(cvb_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, const int32_t* d_seg_ptr,
+                                const int32_t* h_seg_ptr, int n_seg, float thr, float ratio, int32_t* d_match_train,
+                                float* d_match_dist, int32_t* d_n_matches, const uint8_t* xt, const int32_t* seg_tile,
+                                cudaStream_t st) {
+  return knn_dev<HammingMetric, 4>(ctx, d_q, nq, d_t, d_seg_ptr, h_seg_ptr, n_seg, 2, nullptr, nullptr, true, thr, ratio,
+                                   d_match_train, d_match_dist, d_n_matches, st, xt, seg_tile);
+}
+
 // ------------------------------------------------------------------------------------------------
 // C-ABI
 // ------------------------------------------------------------------------------------------------
@@ -921,8 +923,8 @@ int cvb_match_hamming_batch_dev(cvb_ctx* ctx, const uint8_t* d_q, int nq, const 
                                 void* stream) {
   if (!ctx) return CVB_ERR_INVALID;
   CVB_GUARD(ctx);
-  return knn_dev<HammingMetric, 4>(ctx, d_q, nq, d_t, d_seg_ptr, h_seg_ptr, n_seg, 2, nullptr, nullptr, true, thr,
-                                   ratio, d_match_train, d_match_dist, d_n_matches, cvb_stream(ctx, stream));
+  return cvb_match_hamming_tiles_dev(ctx, d_q, nq, d_t, d_seg_ptr, h_seg_ptr, n_seg, thr, ratio, d_match_train, d_match_dist,
+                                     d_n_matches, nullptr, nullptr, cvb_stream(ctx, stream));
 }
 
 int cvb_knn_hamming_batch(cvb_ctx* ctx, const uint8_t* q, int nq, const uint8_t* t, const int32_t* seg_ptr,

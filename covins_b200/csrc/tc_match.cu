@@ -1,28 +1,29 @@
 // tc_match.cu — descriptor k-NN on the 5th-generation tensor cores (tcgen05, kind::i8, accumulators in TMEM).
 //
-// Same contract as scan_kernel in match_kernels.cu (K1 Hamming / K2 L2 / K3 DenseMatcher lists), different bound.
-// The POPC formulation tops out at 16 POPC/clk/SM (measured: 94 % of that roofline).  Here the pairwise term is a
-// u8 x u8 -> s32 GEMM:
-//     Hamming(a,b) = popc(a) + popc(b) - 2 <bits(a), bits(b)>      (bits expanded to 0/1 bytes in shared memory)
-//     |a-b|^2      = |a|^2 + |b|^2 - 2 <a, b>                      (u8 SIFT, exact in s32)
-// issued as tcgen05.mma.cta_group::1.kind::i8 (M = 128 queries, N = 128 train rows, K = 32 bytes per instruction) with
-// the 128x128 s32 accumulator in tensor memory.  One TMEM lane = one query row = one epilogue thread, which receives
-// the train rows of a tile in ascending order — so the per-query selection is the same sequential OpenCV /
-// DenseMatcher rule as in the scalar kernel and the result is bit-identical.
+// Same contract as scan_kernel in match_kernels.cu (K1 Hamming / K2 L2 with the OpenCV k-NN rule, optional fused ratio
+// filter), different bound.  The POPC formulation tops out at 16 POPC/clk/SM (measured: 94 % of that roofline).  Here the
+// pairwise term is an 8-bit GEMM issued as tcgen05.mma.cta_group::1.kind::i8 (M = 128 queries, N = 128 train rows, K = 32
+// bytes per instruction), the query block held in tensor memory for the CTA's lifetime and 128x128 s32 accumulators in
+// tensor memory.  One TMEM lane = one query row = one epilogue thread, which receives the train rows of a segment in
+// ascending order — so the per-query selection is the same sequential OpenCV rule as in the scalar kernel and the result is
+// bit-identical.  A CTA owns one block of 128 queries and streams a contiguous range of candidate segments.  Two kernels:
 //
-// Warp-specialised, persistent CTA (one per SM), 4-stage ring:
-//   warps 0-3  epilogue   wait tmem_full[s] → tcgen05.ld 32x32b.x32 → d = pt[j] - 2 acc (+ pq) → k-list → tmem_empty[s]
-//   warps 4-7  producers  wait empty[s] → read packed rows from HBM (coalesced 16-B loads) → expand / copy into the
-//                         canonical K-major no-swizzle UMMA layout → fence.proxy.async → full[s]
-//   warp 8     MMA        wait full[s], tmem_empty[s] → K/32 x tcgen05.mma → tcgen05.commit → empty[s], tmem_full[s]
-// A CTA owns one block of 128 queries (expanded once, 32 KB of shared memory) and streams a contiguous range of
-// candidate segments.
+// tc_scan_kernel<K>: L2 on u8 SIFT rows, |a-b|^2 = |a|^2 + |b|^2 - 2 <a, b> (exact in s32).  Warp-specialised, persistent
+// (one CTA per SM):
+//   warps 0-15   epilogue   4 column groups x 4 warps: wait tfull[s] → tcgen05.ld 32x32b.x32 → d = |q|^2 + |t|^2 - 2 acc →
+//                           sqrtf key → k-list → tempty[s]; at a segment's end the 4 group lists of a query are merged
+//   warps 16-23  producers  two threads per train row: 16-B loads of the packed rows (two tiles in flight in registers) →
+//                           canonical K-major no-swizzle UMMA layout in a 4-stage ring + row norms → fence.proxy.async → full[s]
+//   warp 24      MMA        wait full[s] and a free accumulator → 4 x tcgen05.mma into a 3-stage TMEM ring → tcgen05.commit
+//
+// xt::tc_xt_kernel<K>: Hamming on 256-bit ORB rows from operand tiles expanded once, with the distance folded into the GEMM
+// (namespace xt below).
 #include <float.h>
 #include <limits.h>
-#include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "cvb_internal.cuh"
@@ -32,7 +33,7 @@ namespace cvb_tc {
 
 constexpr int TM = 128;       // queries per CTA (UMMA M)
 constexpr int TN = 128;       // train rows per tile (UMMA N)
-constexpr int STAGES = 4;        // shared-memory ring of expanded train tiles
+constexpr int STAGES = 4;        // shared-memory ring of train tiles
 constexpr int ACC_STAGES = 3;    // TMEM ring of 128-column accumulators: columns [0, 384); the query operand sits at column 384
 constexpr uint32_t A_COL = ACC_STAGES * 128;
 constexpr int NORM_RING = 8;
@@ -101,18 +102,7 @@ __device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&r)[32]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-// 32 lanes x 32 columns, the low 16 bits of two adjacent columns packed into one register (even column low, odd column high)
-__device__ __forceinline__ void tc_ld32_pack16(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.pack::16b.x16.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-        "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// 32 lanes x 128 columns as 64 packed registers
+// 32 lanes x 128 columns, the low 16 bits of two adjacent columns packed into one register (even column low, odd column high)
 __device__ __forceinline__ void tc_ld64_pack16(uint32_t taddr, uint32_t (&r)[64]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.pack::16b.x64.b32 "
@@ -148,89 +138,6 @@ __device__ __forceinline__ uint4 ldg_nc(const void* p) {
   asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
   return r;
 }
-
-// ---- metrics: how a packed row becomes a K-major operand row, and its additive norm term ----------------------
-// A row is handled by TWO threads (half = 0/1), each loading kLoads 16-byte pieces of the packed row (so that the loads
-// of several tiles can be kept in flight in registers) and writing its share of the operand chunks.
-struct TcHamming {
-  static constexpr int kRowBytes = 32;    // packed bytes in HBM
-  static constexpr int kKBytes = 256;     // operand bytes (one byte per bit)
-  static constexpr int kLoads = 1;        // uint4 per half row
-  static constexpr int kPrefetch = 3;     // tiles in flight per producer thread
-  static constexpr bool kIsL2 = false;
-  static __device__ __forceinline__ void load_half(const uint8_t* __restrict__ row, int half, uint4 (&v)[kLoads]) {
-    v[0] = ldg_nc(row + 16 * half);
-  }
-  // writes operand chunks 8 half .. 8 half + 7 of the row and returns the partial popcount
-  static __device__ __forceinline__ int store_half(const uint4 (&v)[kLoads], int half, uint8_t* dst_row0) {
-    const uint32_t w[4] = {v[0].x, v[0].y, v[0].z, v[0].w};
-    int pc = 0;
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-      pc += __popc(w[i]);
-      // byte j of output word k is 0x80 if bit (k + 8 j) of w[i] is set, else 0 (the same permutation and the same
-      // 0/128 encoding on both operands → accumulator = 16384 * popc(a & b)).  The left shift is a multiply so that it
-      // issues on the FMA pipe; only the mask uses the (narrower) ALU pipe.
-      uint4 lo, hi;
-      lo.x = (w[i] * 128u) & 0x80808080u; lo.y = (w[i] * 64u) & 0x80808080u; lo.z = (w[i] * 32u) & 0x80808080u; lo.w = (w[i] * 16u) & 0x80808080u;
-      hi.x = (w[i] * 8u) & 0x80808080u; hi.y = (w[i] * 4u) & 0x80808080u; hi.z = (w[i] * 2u) & 0x80808080u; hi.w = w[i] & 0x80808080u;
-      *reinterpret_cast<uint4*>(dst_row0 + (8 * half + 2 * i) * 128) = lo;
-      *reinterpret_cast<uint4*>(dst_row0 + (8 * half + 2 * i + 1) * 128) = hi;
-    }
-    return pc;
-  }
-  // query side (tensor memory, one thread per row): the same K permutation with 0/1 bytes, so that accumulator =
-  // 128 * popc(a & b) = (2 popc(a & b)) << 6, which is what the packed 16-bit keys of the epilogue subtract.  Packed word i
-  // of the row becomes operand bytes [32 i, 32 i + 32) = one K = 32 instruction = 8 TMEM columns.
-  static constexpr int kQWords = 8;   // 32-byte operand groups per row
-  static __device__ __forceinline__ int load_q(const uint8_t* __restrict__ row, uint32_t (&w)[8]) {
-    const uint4 a = ldg_nc(row), b = ldg_nc(row + 16);
-    w[0] = a.x; w[1] = a.y; w[2] = a.z; w[3] = a.w; w[4] = b.x; w[5] = b.y; w[6] = b.z; w[7] = b.w;
-    int pc = 0;
-#pragma unroll
-    for (int i = 0; i < 8; i++) pc += __popc(w[i]);
-    return pc;
-  }
-  static __device__ __forceinline__ void expand_q(const uint32_t (&w)[8], int i, uint32_t (&r)[8]) {
-#pragma unroll
-    for (int b = 0; b < 8; b++) r[b] = (w[i] >> b) & 0x01010101u;
-  }
-};
-struct TcL2 {
-  static constexpr int kRowBytes = 128;
-  static constexpr int kKBytes = 128;
-  static constexpr int kLoads = 4;
-  static constexpr int kPrefetch = 2;
-  static constexpr bool kIsL2 = true;
-  static __device__ __forceinline__ void load_half(const uint8_t* __restrict__ row, int half, uint4 (&v)[kLoads]) {
-#pragma unroll
-    for (int c = 0; c < 4; c++) v[c] = ldg_nc(row + 64 * half + 16 * c);
-  }
-  static __device__ __forceinline__ int store_half(const uint4 (&v)[kLoads], int half, uint8_t* dst_row0) {
-    unsigned n2 = 0;
-#pragma unroll
-    for (int c = 0; c < 4; c++) {
-      n2 = __dp4a(v[c].x, v[c].x, n2); n2 = __dp4a(v[c].y, v[c].y, n2); n2 = __dp4a(v[c].z, v[c].z, n2); n2 = __dp4a(v[c].w, v[c].w, n2);
-      *reinterpret_cast<uint4*>(dst_row0 + (4 * half + c) * 128) = v[c];
-    }
-    return (int)n2;
-  }
-  static constexpr int kQWords = 4;   // 128 operand bytes per row = 4 groups of 32
-  static __device__ __forceinline__ int load_q(const uint8_t* __restrict__ row, uint32_t (&w)[32]) {
-    unsigned n2 = 0;
-#pragma unroll
-    for (int c = 0; c < 8; c++) {
-      const uint4 v = ldg_nc(row + 16 * c);
-      w[4 * c] = v.x; w[4 * c + 1] = v.y; w[4 * c + 2] = v.z; w[4 * c + 3] = v.w;
-      n2 = __dp4a(v.x, v.x, n2); n2 = __dp4a(v.y, v.y, n2); n2 = __dp4a(v.z, v.z, n2); n2 = __dp4a(v.w, v.w, n2);
-    }
-    return (int)n2;
-  }
-  static __device__ __forceinline__ void expand_q(const uint32_t (&w)[32], int i, uint32_t (&r)[8]) {
-#pragma unroll
-    for (int b = 0; b < 8; b++) r[b] = w[8 * i + b];
-  }
-};
 
 // k-list of (key, idx) kept sorted ascending by (key, idx); OpenCV rule for a stream with ascending idx:
 // enter iff key < worst key; placed after all entries with key <= new key.
@@ -269,35 +176,27 @@ constexpr int PROD_WARP0 = EPI_THREADS / 32;    // producer warps 16..23 (two th
 constexpr int PROD_THREADS = 256;
 constexpr int MMA_WARP = PROD_WARP0 + PROD_THREADS / 32;   // warp 24
 constexpr int NUM_THREADS = (MMA_WARP + 1) * 32;
+constexpr int KB = 128;                         // bytes per SIFT row = operand bytes per row (u8, used as they are)
+constexpr int PF = 2;                           // tiles in flight per producer thread
 
-template <class M, int K>
+template <int K>
 constexpr size_t smem_bytes() {
-  return (size_t)STAGES * TN * M::kKBytes + (size_t)NORM_RING * TN * sizeof(int) +
+  return (size_t)STAGES * TN * KB + (size_t)NORM_RING * TN * sizeof(int) +
          (size_t)2 * TM * GROUPS * K * 2 * sizeof(int) + 64 * sizeof(uint64_t);
 }
 
-// operand row r of a tile with KB operand bytes per row: byte offset of its chunk 0
-template <int KB>
+// operand row r of a tile: byte offset of its chunk 0
 __device__ __forceinline__ uint32_t row_offset(int r) {
   return (uint32_t)(r >> 3) * (KB * 8) + (uint32_t)(r & 7) * 16;
 }
 
-// keys: Hamming → the distance; L2 → the bit pattern of sqrtf(d2) (non-negative floats order like their bits), which
-// is what OpenCV compares.  kInfKey is larger than any real key of either kind.
+// keys: the bit pattern of sqrtf(d2) (non-negative floats order like their bits), which is what OpenCV compares.  kInfKey
+// is larger than any real key.
 constexpr int kInfKey = 0x7F000000;
 
-// development trace (COVINS_B200_TC_DEBUG bit 16): clock64 stamps of CTA 0's first tiles, per role
-constexpr int TRACE_TILES = 48;
-__device__ long long g_tc_trace[3][TRACE_TILES][4];
-#define TC_STAMP(role, n, slot)                                                                                 \
-  do {                                                                                                          \
-    if ((p.dbg & 16) && blockIdx.x == 0 && (n) < TRACE_TILES) g_tc_trace[role][n][slot] = clock64();            \
-  } while (0)
-
-template <class M, int K>
+template <int K>
 __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
-  constexpr int KB = M::kKBytes;
   uint8_t* sB = smem;
   int* sNorm = reinterpret_cast<int*>(sB + (size_t)STAGES * TN * KB);
   int* sList = sNorm + NORM_RING * TN;                       // [2][TM][GROUPS][K][2]
@@ -335,22 +234,23 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams 
     // the query block → tensor memory: thread = row = TMEM lane (warps 0-3 own lanes 32 w .. 32 w + 31), 8 columns
     // (= one K = 32 instruction's worth) per tcgen05.st
     const int q = qb * TM + tid;
-    uint32_t w[M::kIsL2 ? 32 : 8];
-    int nrm = 0;
+    uint32_t w[32];
+    unsigned nrm = 0;
     if (q < p.nq) {
-      nrm = M::load_q(p.q + (size_t)q * M::kRowBytes, w);
+#pragma unroll
+      for (int c = 0; c < 8; c++) {
+        const uint4 v = ldg_nc(p.q + (size_t)q * KB + 16 * c);
+        w[4 * c] = v.x; w[4 * c + 1] = v.y; w[4 * c + 2] = v.z; w[4 * c + 3] = v.w;
+        nrm = __dp4a(v.x, v.x, nrm); nrm = __dp4a(v.y, v.y, nrm); nrm = __dp4a(v.z, v.z, nrm); nrm = __dp4a(v.w, v.w, nrm);
+      }
     } else {
 #pragma unroll
-      for (int i = 0; i < (M::kIsL2 ? 32 : 8); i++) w[i] = 0;
+      for (int i = 0; i < 32; i++) w[i] = 0;
     }
-    sQNorm[tid] = nrm;
+    sQNorm[tid] = (int)nrm;
     const uint32_t a_taddr = tmem_base + ((uint32_t)(warp * 32) << 16) + A_COL;
 #pragma unroll
-    for (int i = 0; i < KB / 32; i++) {
-      uint32_t r[8];
-      M::expand_q(w, i, r);
-      tc_st8(a_taddr + 8 * i, r);
-    }
+    for (int i = 0; i < KB / 32; i++) tc_st8(a_taddr + 8 * i, w + 8 * i);
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
   }
   tc_fence_before();
@@ -359,8 +259,8 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams 
 
   if (warp >= PROD_WARP0 && warp < MMA_WARP) {
     // =================================== producers ===================================
-    // Two threads per train row; the packed rows of the next kPrefetch tiles are held in registers so that the HBM
-    // latency (~1 us) of a tile overlaps the expansion of the previous ones.
+    // Two threads per train row, 64 bytes each; the packed rows of the next PF tiles are held in registers so that the
+    // HBM latency (~1 us) of a tile overlaps the stores of the previous ones.
     const int pt = tid - PROD_WARP0 * 32;   // 0..255
     const int prow = (pt & 7) | ((pt >> 4) << 3), half = (pt >> 3) & 1;
     struct TileIt {
@@ -381,12 +281,15 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams 
     TileIt it{seg0 - 1, 0, 0, 0, seg1, p.seg_ptr, false}, ld = it;
     it.next_seg();
     ld.next_seg();
-    constexpr int PF = M::kPrefetch;
-    uint4 pf[PF][M::kLoads];
-    auto issue_load = [&](uint4 (&v)[M::kLoads]) {
+    uint4 pf[PF][4];
+    auto issue_load = [&](uint4 (&v)[4]) {
       if (!ld.done) {
         const int row = ld.r0 + prow;
-        if (row < ld.len) M::load_half(p.t + (size_t)(ld.s_begin + row) * M::kRowBytes, half, v);
+        if (row < ld.len) {
+          const uint8_t* src = p.t + (size_t)(ld.s_begin + row) * KB + 64 * half;
+#pragma unroll
+          for (int c = 0; c < 4; c++) v[c] = ldg_nc(src + 16 * c);
+        }
         ld.advance();
       }
     };
@@ -397,38 +300,33 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams 
 #pragma unroll
       for (int u = 0; u < PF; u++) {
         if (it.done) break;
-        uint4 cur[M::kLoads];
+        uint4 cur[4];
 #pragma unroll
-        for (int c = 0; c < M::kLoads; c++) cur[c] = pf[u][c];
+        for (int c = 0; c < 4; c++) cur[c] = pf[u][c];
         issue_load(pf[u]);   // refill this register slot with the tile PF steps ahead
         const int s = n % STAGES;
-        if (pt == 0) TC_STAMP(0, n, 0);
         if (n >= STAGES) cvb_mbar_wait(&empty[s], ((n / STAGES) - 1) & 1);
-        if (pt == 0) TC_STAMP(0, n, 1);
-        uint8_t* dst = sB + (size_t)s * TN * KB + row_offset<KB>(prow);
+        uint8_t* dst = sB + (size_t)s * TN * KB + row_offset(prow);
         const bool rv = it.r0 + prow < it.len;
-        int part = 0;
-        if (rv && !(p.dbg & 2)) {
-          part = M::store_half(cur, half, dst);
+        int part = 0;   // |row|^2 over this thread's half
+        if (rv) {
+          unsigned n2 = 0;
+#pragma unroll
+          for (int c = 0; c < 4; c++) {
+            n2 = __dp4a(cur[c].x, cur[c].x, n2); n2 = __dp4a(cur[c].y, cur[c].y, n2); n2 = __dp4a(cur[c].z, cur[c].z, n2); n2 = __dp4a(cur[c].w, cur[c].w, n2);
+            *reinterpret_cast<uint4*>(dst + (4 * half + c) * 128) = cur[c];
+          }
+          part = (int)n2;
         } else {
-          for (int c = 0; c < KB / 32; c++) *reinterpret_cast<uint4*>(dst + (half * (KB / 32) + c) * 128) = make_uint4(0, 0, 0, 0);
+          for (int c = 0; c < 4; c++) *reinterpret_cast<uint4*>(dst + (4 * half + c) * 128) = make_uint4(0, 0, 0, 0);
         }
         part += __shfl_xor_sync(0xffffffffu, part, 8);   // the two halves of a row sit 8 lanes apart
-        // Hamming: packed column term (popc(row) << 22 | segment-local index), L2: |row|^2; tail rows never enter a list
-        if (M::kIsL2) {
-          if (half == 0) sNorm[(n % NORM_RING) * TN + prow] = rv ? part : kInf;
-        } else if (half == 0) {
-          // Hamming: 16-bit column term ((popc(row) + 256) << 6 | column within its 32-column group); 0xFFFF = no row
-          reinterpret_cast<uint16_t*>(sNorm)[(n % NORM_RING) * TN + prow] =
-              rv ? (uint16_t)(((part + 256) << 6) | (prow & 31)) : (uint16_t)0xFFFFu;
-        }
+        if (half == 0) sNorm[(n % NORM_RING) * TN + prow] = rv ? part : kInf;   // tail rows never enter a list
         // every lane makes its own stores visible to the async proxy; ONE arrival per warp (hundreds of same-address
         // mbarrier arrivals per tile serialise in shared memory and cost more than the tile's MMAs)
-        if (pt == 0) TC_STAMP(0, n, 2);
         fence_proxy_async();
         __syncwarp();
         if (lane == 0) mbar_arrive(&full[s]);
-        if (pt == 0) TC_STAMP(0, n, 3);
         it.advance();
         n++;
       }
@@ -444,13 +342,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams 
     int n = 0;
     for (int seg = seg0; seg < seg1; seg++) {
       const int len = __shfl_sync(0xffffffffu, p.seg_ptr[seg + 1] - p.seg_ptr[seg], 0);
+#pragma unroll 2   // left alone, the compiler unrolls this small body 4x and emits 7 copies of the issue sequence
       for (int r0 = 0; r0 < len; r0 += TN, n++) {
         const int s = n % STAGES, ts = n % ACC_STAGES;
-        if (lane == 0) TC_STAMP(1, n, 0);
         cvb_mbar_wait(&full[s], (n / STAGES) & 1);
-        if (lane == 0) TC_STAMP(1, n, 1);
         if (n >= ACC_STAGES) cvb_mbar_wait(&tempty[ts], ((n / ACC_STAGES) - 1) & 1);
-        if (lane == 0) TC_STAMP(1, n, 2);
         tc_fence_after();
         const uint64_t b_desc0 = make_desc(b_addr0 + (uint32_t)s * (TN * KB), 128, KB * 8);
         const uint32_t d_tmem = tmem_base + (uint32_t)ts * TN;
@@ -461,7 +357,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams 
           tc_commit(&empty[s]);    // shared-memory slot reusable once these MMAs have read it
           tc_commit(&tfull[ts]);   // accumulator ready
         }
-        if (lane == 0) TC_STAMP(1, n, 3);
         __syncwarp();
       }
     }
@@ -477,145 +372,60 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams 
     for (int seg = seg0; seg < seg1; seg++, segc++) {
       const int len = p.seg_ptr[seg + 1] - p.seg_ptr[seg];
 #pragma unroll
-      for (int c = 0; c < K; c++) { wk[c] = M::kIsL2 ? kInfKey : INT_MAX; wi[c] = -1; wd2[c] = kInf; }
+      for (int c = 0; c < K; c++) { wk[c] = kInfKey; wi[c] = -1; wd2[c] = kInf; }
       for (int r0 = 0; r0 < len; r0 += TN, n++) {
         const int s = n % ACC_STAGES;
-        if (tid == 0) TC_STAMP(2, n, 0);
         cvb_mbar_wait(&tfull[s], (n / ACC_STAGES) & 1);
-        if (tid == 0) TC_STAMP(2, n, 1);
         tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)s * TN + grp * 32;
         uint32_t acc[32];
-        // Hamming: the accumulator 128 * popc(q & t) <= 32768 fits 16 bits, so two adjacent columns are read as ONE packed
-        // register (LDTM.x16.PACK16BIT: even column low, odd column high) — exactly the layout of the packed 16-bit keys
-        const bool pack16 = !M::kIsL2 && !(p.dbg & 8);   // dbg 8: the unpacked read (development comparison)
-        if (p.dbg & 4) {
+        tc_ld32(taddr, acc);
+        if (valid) {
+          const int4* nrm4 = reinterpret_cast<const int4*>(sNorm + (n % NORM_RING) * TN + grp * 32);
 #pragma unroll
-          for (int i = 0; i < 32; i++) acc[i] = 0;      // experiment: no TMEM read at all (results invalid)
-        } else if (pack16) {
-          tc_ld32_pack16(taddr, acc);
-        } else {
-          tc_ld32(taddr, acc);
-        }
-        if (valid && !(p.dbg & 1)) {
-          if (!M::kIsL2) {
-            // Two columns per instruction: 16-bit keys ((popc(t) - 2 popc(q & t) + 256) << 6 | column) packed pairwise
-            // (even column low, odd column high), k-lists kept per half with packed 16-bit min/max (VIMNMX.U16x2 issues
-            // at the 32-bit rate), merged into the 32-bit (distance, index) lists once per tile — and only if the tile
-            // holds a candidate that beats the current k-th entry (later tiles have larger indices, so "beats" is a
-            // strict distance comparison).
-            const uint4* nrm4 = reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(sNorm) + (n % NORM_RING) * TN + grp * 32);
-            unsigned pk[K];
+          for (int i4 = 0; i4 < 8; i4++) {
+            const int4 nn = nrm4[i4];
+            const int nv[4] = {nn.x, nn.y, nn.z, nn.w};
 #pragma unroll
-            for (int c = 0; c < K; c++) pk[c] = 0xFFFFFFFFu;
-#pragma unroll
-            for (int i4 = 0; i4 < 4; i4++) {
-              const uint4 nn = nrm4[i4];
-              const unsigned nv[4] = {nn.x, nn.y, nn.z, nn.w};
-#pragma unroll
-              for (int j = 0; j < 4; j++) {
-                const int i = 8 * i4 + 2 * j;   // columns i (low half) and i + 1 (high half)
-                unsigned x = pack16 ? nv[j] - acc[4 * i4 + j] : nv[j] + acc[i] * 0xFFFFFFFFu + acc[i + 1] * 0xFFFF0000u;
-#pragma unroll
-                for (int c = 0; c < K; c++) {
-                  const unsigned lo = __vminu2(pk[c], x);
-                  x = __vmaxu2(pk[c], x);
-                  pk[c] = lo;
-                }
-              }
-            }
-            const unsigned best16 = min(pk[0] & 0xFFFFu, pk[0] >> 16);
-            const int worst_v = wk[K - 1] == INT_MAX ? 1024 : (wk[K - 1] >> kIdxBits) + 256;   // arithmetic shift: t-domain value
-            if ((int)(best16 >> 6) < worst_v) {
-#pragma unroll
-              for (int c = 0; c < K; c++)
-#pragma unroll
-                for (int h = 0; h < 2; h++) {
-                  const unsigned k16 = h ? (pk[c] >> 16) : (pk[c] & 0xFFFFu);
-                  int x = k16 == 0xFFFFu ? INT_MAX
-                                         : (int)((((unsigned)(k16 >> 6) - 256u) << kIdxBits) + (unsigned)(r0 + grp * 32 + (int)(k16 & 63u)));
-#pragma unroll
-                  for (int cc = 0; cc < K; cc++) {
-                    const int lo = min(wk[cc], x);
-                    x = max(wk[cc], x);
-                    wk[cc] = lo;
-                  }
-                }
-            }
-          } else {
-            const int4* nrm4 = reinterpret_cast<const int4*>(sNorm + (n % NORM_RING) * TN + grp * 32);
-#pragma unroll
-            for (int i4 = 0; i4 < 8; i4++) {
-              const int4 nn = nrm4[i4];
-              const int nv[4] = {nn.x, nn.y, nn.z, nn.w};
-#pragma unroll
-              for (int j = 0; j < 4; j++) {
-                const int i = 4 * i4 + j;
-                const int d = qn + nv[j] - 2 * (int)acc[i];
-                if (d < wd2[K - 1]) {
-                  const int key = __float_as_int(__fsqrt_rn((float)d));
-                  if (key < wk[K - 1]) {
-                    insert_key<K>(wk, wi, key, r0 + grp * 32 + i);
-                    const float f = __int_as_float(wk[K - 1]);   // raw-distance bound of the worst entry (pre-test)
-                    wd2[K - 1] = wk[K - 1] == kInfKey ? kInf : (int)ceilf(f * f * 1.000001f) + 1;
-                  }
+            for (int j = 0; j < 4; j++) {
+              const int i = 4 * i4 + j;
+              const int d = qn + nv[j] - 2 * (int)acc[i];
+              if (d < wd2[K - 1]) {
+                const int key = __float_as_int(__fsqrt_rn((float)d));
+                if (key < wk[K - 1]) {
+                  insert_key<K>(wk, wi, key, r0 + grp * 32 + i);
+                  const float f = __int_as_float(wk[K - 1]);   // raw-distance bound of the worst entry (pre-test)
+                  wd2[K - 1] = wk[K - 1] == kInfKey ? kInf : (int)ceilf(f * f * 1.000001f) + 1;
                 }
               }
             }
           }
         }
-        if (tid == 0) TC_STAMP(2, n, 2);
+        // accumulator and norms consumed: the MMA warp may overwrite this TMEM stage
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&tempty[s]);
-        if (tid == 0) TC_STAMP(2, n, 3);   // accumulator and norms consumed: the MMA warp may overwrite this TMEM stage
       }
       // ---- segment finished: combine the 4 column-group lists of each query (k smallest by (key, idx)) ----
       int* lst = sList + (size_t)(segc & 1) * TM * GROUPS * K * 2;
-      if (!M::kIsL2) {
-        const int qq = qn << kIdxBits;
 #pragma unroll
-        for (int c = 0; c < K; c++) lst[(row * GROUPS + grp) * K + c] = wk[c] == INT_MAX ? INT_MAX : wk[c] + qq;
-      } else {
-#pragma unroll
-        for (int c = 0; c < K; c++) {
-          lst[((row * GROUPS + grp) * K + c) * 2 + 0] = wk[c];
-          lst[((row * GROUPS + grp) * K + c) * 2 + 1] = wi[c];
-        }
+      for (int c = 0; c < K; c++) {
+        lst[((row * GROUPS + grp) * K + c) * 2 + 0] = wk[c];
+        lst[((row * GROUPS + grp) * K + c) * 2 + 1] = wi[c];
       }
       asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");
       if (grp == 0) {
-        float fd[K];   // final distances as float (DMatch::distance)
-        if (!M::kIsL2) {
 #pragma unroll
-          for (int c = 0; c < K; c++) wk[c] = INT_MAX;
-          for (int e = 0; e < GROUPS * K; e++) {
-            int x = lst[row * GROUPS * K + e];
-#pragma unroll
-            for (int c = 0; c < K; c++) {
-              const int lo = min(wk[c], x);
-              x = max(wk[c], x);
-              wk[c] = lo;
-            }
-          }
+        for (int c = 0; c < K; c++) { wk[c] = kInfKey; wi[c] = -1; }
+        for (int g2 = 0; g2 < GROUPS; g2++)
 #pragma unroll
           for (int c = 0; c < K; c++) {
-            wi[c] = wk[c] == INT_MAX ? -1 : (wk[c] & ((1 << kIdxBits) - 1));
-            wk[c] = wk[c] == INT_MAX ? INT_MAX : (wk[c] >> kIdxBits);
-            fd[c] = (float)wk[c];
+            const int kk = lst[((row * GROUPS + g2) * K + c) * 2], ii = lst[((row * GROUPS + g2) * K + c) * 2 + 1];
+            if (ii >= 0) insert_lex<K>(wk, wi, kk, ii);
           }
-        } else {
+        float fd[K];   // final distances as float (DMatch::distance)
 #pragma unroll
-          for (int c = 0; c < K; c++) { wk[c] = kInfKey; wi[c] = -1; }
-          for (int g2 = 0; g2 < GROUPS; g2++)
-#pragma unroll
-            for (int c = 0; c < K; c++) {
-              const int kk = lst[((row * GROUPS + g2) * K + c) * 2], ii = lst[((row * GROUPS + g2) * K + c) * 2 + 1];
-              if (ii >= 0) insert_lex<K>(wk, wi, kk, ii);
-            }
-#pragma unroll
-          for (int c = 0; c < K; c++) fd[c] = __int_as_float(wk[c]);
-        }
+        for (int c = 0; c < K; c++) fd[c] = __int_as_float(wk[c]);
         if (p.filter) {
           bool ok = false;
           if (K >= 2 && valid) {
@@ -632,8 +442,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams 
 #pragma unroll
           for (int c = 0; c < K; c++) {
             p.out_idx[o + c] = wi[c];
-            if (M::kIsL2) reinterpret_cast<float*>(p.out_dist)[o + c] = wi[c] >= 0 ? fd[c] : FLT_MAX;
-            else reinterpret_cast<int32_t*>(p.out_dist)[o + c] = wi[c] >= 0 ? wk[c] : INT_MAX;
+            reinterpret_cast<float*>(p.out_dist)[o + c] = wi[c] >= 0 ? fd[c] : FLT_MAX;
           }
         }
       }
@@ -648,20 +457,21 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_scan_kernel(const TcParams 
   }
 }
 
-
 // ===================================================================================================================
 // Hamming k-NN on PRE-EXPANDED operand tiles.
 //
-// The kernel above spends its issue slots on ALU work: producers turn every packed bit into a byte (>= 64 logic
-// operations per row and tile) and the epilogue rebuilds the distance from the accumulator and a per-column term read
-// from shared memory.  Both disappear when the operand the tensor core reads is stored once and reused by every query:
+// Hamming(a,b) = popc(a) + popc(b) - 2 popc(a & b), and popc(a & b) is an 8-bit GEMM once the 256 bits of a row are
+// expanded to bytes.  Expanding inside the matching kernel costs >= 64 logic operations per row and tile, and rebuilding
+// the distance from the accumulator costs ALU work per pair in the epilogue: the ALU, not the tensor pipe, then bounds
+// the kernel.  Both disappear when the operand the tensor core reads is stored once and reused by every query:
 //
 //   * cvb_tc::expand_tiles writes, per keyframe, ceil(rows / 128) tiles of 128 rows x 288 operand bytes in exactly the
 //     shared-memory image tcgen05.mma wants (K-major, no swizzle, 8-row groups of 2304 B): 256 data bytes (0x80 = -128
 //     as s8 for a set bit) + a 32-byte KEY slice.  A tile is 36 KB and contiguous, so the producer is ONE thread issuing
 //     cp.async.bulk copies (TMA engine) — no register path, no expansion in the matching kernel.  The map database
 //     (map_db.cu) keeps these tiles resident next to the packed rows; 9 bytes of HBM per descriptor byte, read at
-//     ~2 TB/s by a kernel that is bound by the tensor pipe, not by HBM.
+//     ~2 TB/s by a kernel that is bound by the tensor pipe, not by HBM.  A train set without resident tiles (the
+//     raw-pointer API) is expanded into the workspace by launch() before the matching kernel runs.
 //   * the key slice folds the whole distance into the GEMM: with query bytes 0/2 (u8) and
 //         A key bytes = [1, 128, 128, 128, c4, c5, c6, 0...]   c4 + c5 + c6 = 2 popc(q)      (per query row)
 //         B key bytes = [col, p1, p2, p3, 64, 64, 64, 0...]    p1 + p2 + p3 = popc(t)        (per train row)
@@ -685,11 +495,40 @@ constexpr int MMA_WARP_X = EPI_WARPS + 1;
 constexpr int XTHREADS = (MMA_WARP_X + 1) * 32;
 constexpr uint32_t XA_COL = NGRP * 128;       // query operand: TMEM columns [384, 456)
 constexpr int kKeyInvalid = 32896;            // keys >= this are "no row"
-constexpr int kPaceWindow = 96;               // tiles a CTA may run ahead of the slowest CTA of its keyframe range (3.4 MB)
-constexpr long kPaceMinTiles = 1536;          // pacing only when a CTA walks more tiles than this
 constexpr size_t kSmemBytes = (size_t)XSTAGES * TILE_BYTES + 1024;
 
 __device__ __forceinline__ uint32_t xrow_off(int r) { return (uint32_t)(r >> 3) * (KX * 8) + (uint32_t)(r & 7) * 16; }
+
+// ---- packed 256-bit rows (32 bytes) ----
+// train side: a row is expanded by TWO threads (half = 0/1), 16 packed bytes each
+__device__ __forceinline__ uint4 load_half(const uint8_t* __restrict__ row, int half) { return ldg_nc(row + 16 * half); }
+// writes operand chunks 8 half .. 8 half + 7 of the row and returns the partial popcount
+__device__ __forceinline__ int store_half(const uint4 v, int half, uint8_t* dst_row0) {
+  const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+  int pc = 0;
+#pragma unroll
+  for (int i = 0; i < 4; i++) {
+    pc += __popc(w[i]);
+    // byte j of output word k is 0x80 (-128 as s8) if bit (k + 8 j) of w[i] is set, else 0; the query side uses the same
+    // permutation with 0/2 bytes (tc_xt_kernel).  The left shift is a multiply so that it issues on the FMA pipe; only
+    // the mask uses the (narrower) ALU pipe.
+    uint4 lo, hi;
+    lo.x = (w[i] * 128u) & 0x80808080u; lo.y = (w[i] * 64u) & 0x80808080u; lo.z = (w[i] * 32u) & 0x80808080u; lo.w = (w[i] * 16u) & 0x80808080u;
+    hi.x = (w[i] * 8u) & 0x80808080u; hi.y = (w[i] * 4u) & 0x80808080u; hi.z = (w[i] * 2u) & 0x80808080u; hi.w = w[i] & 0x80808080u;
+    *reinterpret_cast<uint4*>(dst_row0 + (8 * half + 2 * i) * 128) = lo;
+    *reinterpret_cast<uint4*>(dst_row0 + (8 * half + 2 * i + 1) * 128) = hi;
+  }
+  return pc;
+}
+// query side (one thread per row): the 8 packed words and the row's popcount
+__device__ __forceinline__ int load_q(const uint8_t* __restrict__ row, uint32_t (&w)[8]) {
+  const uint4 a = ldg_nc(row), b = ldg_nc(row + 16);
+  w[0] = a.x; w[1] = a.y; w[2] = a.z; w[3] = a.w; w[4] = b.x; w[5] = b.y; w[6] = b.z; w[7] = b.w;
+  int pc = 0;
+#pragma unroll
+  for (int i = 0; i < 8; i++) pc += __popc(w[i]);
+  return pc;
+}
 
 // ---- one-time expansion (also the append path of the map database) ----
 __global__ void __launch_bounds__(256) expand_tiles_kernel(const uint8_t* __restrict__ t, const int32_t* __restrict__ seg_ptr,
@@ -707,9 +546,7 @@ __global__ void __launch_bounds__(256) expand_tiles_kernel(const uint8_t* __rest
   uint8_t* dst = out + (size_t)tile * TILE_BYTES + xrow_off(prow);
   int part = 0;
   if (rv) {
-    uint4 v[1];
-    TcHamming::load_half(t + (size_t)(s_begin + r0 + prow) * 32, half, v);
-    part = TcHamming::store_half(v, half, dst);
+    part = store_half(load_half(t + (size_t)(s_begin + r0 + prow) * 32, half), half, dst);
   } else {
 #pragma unroll
     for (int c = 0; c < 8; c++) *reinterpret_cast<uint4*>(dst + (8 * half + c) * 128) = make_uint4(0, 0, 0, 0);
@@ -789,7 +626,7 @@ __global__ void __launch_bounds__(XTHREADS, 1) tc_xt_kernel(const TcParams p) {
     uint32_t w[8];
     int pq = 0;
     if (q < p.nq) {
-      pq = TcHamming::load_q(p.q + (size_t)q * 32, w);
+      pq = load_q(p.q + (size_t)q * 32, w);
     } else {
 #pragma unroll
       for (int i = 0; i < 8; i++) w[i] = 0;
@@ -825,22 +662,6 @@ __global__ void __launch_bounds__(XTHREADS, 1) tc_xt_kernel(const TcParams p) {
         for (int g = 0; g < NGRP; g++) {
           if (!S.active(g)) continue;
           const int s = n % XSTAGES;
-          if (p.progress != nullptr && (n & 15) == 0 && n > 0) {
-            // Pacing (large maps only): the nqb CTAs that walk the same keyframe range read every tile once from HBM and
-            // nqb - 1 times from L2 — as long as they stay within an L2's worth of each other.  Over thousands of tiles they
-            // drift apart (C5: 4448 tiles per CTA → 8x the HBM traffic, 4.8x the time); the producer therefore publishes its
-            // position every 16 tiles and waits while it is more than kPaceWindow tiles ahead of the slowest CTA of its group.
-            // (All CTAs are resident — grid <= SM count, one CTA per SM — so the wait cannot deadlock.)
-            volatile int* grp_prog = p.progress + (size_t)part * p.nqb;
-            grp_prog[qb] = n;
-            __threadfence();
-            for (;;) {
-              int mn = INT_MAX;
-              for (int i = 0; i < p.nqb; i++) mn = min(mn, grp_prog[i]);
-              if (mn + kPaceWindow >= n) break;
-              __nanosleep(500);
-            }
-          }
           if (n >= XSTAGES) cvb_mbar_wait(&empty[s], ((n / XSTAGES) - 1) & 1);
           cvb_mbar_expect_tx(&full[s], TILE_BYTES);
           const uint8_t* src = p.xt + (size_t)(S.tile0[g] + S.t[g]) * TILE_BYTES;
@@ -850,10 +671,6 @@ __global__ void __launch_bounds__(XTHREADS, 1) tc_xt_kernel(const TcParams p) {
           S.advance(g);
           n++;
         }
-      }
-      if (p.progress != nullptr) {   // done: never hold the others back
-        reinterpret_cast<volatile int*>(p.progress)[(size_t)part * p.nqb + qb] = INT_MAX;
-        __threadfence();
       }
     }
     __syncwarp();
@@ -910,7 +727,7 @@ __global__ void __launch_bounds__(XTHREADS, 1) tc_xt_kernel(const TcParams p) {
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&tempty[g]);   // accumulator in registers: the MMA warp may start this stream's next tile
-        if (valid && !(p.dbg & 1)) {
+        if (valid) {
           unsigned pk[K];
 #pragma unroll
           for (int c = 0; c < K; c++) pk[c] = 0xFFFFFFFFu;
@@ -984,16 +801,7 @@ __global__ void __launch_bounds__(XTHREADS, 1) tc_xt_kernel(const TcParams p) {
 }
 
 template <int K>
-int launch_xt(cvb_ctx* ctx, TcParams p, long total_tiles, cudaStream_t st) {
-  p.progress = nullptr;
-  // opt-in (COVINS_B200_TC_PACING=1): at C5 size the standalone request runs at full speed without it (1.77 ms, 5.6 Tpairs/s) and 6 %
-  // slower with it; it is kept for the case the CTAs of a keyframe range do drift out of each other's L2 window
-  const char* pace = getenv("COVINS_B200_TC_PACING");
-  if (p.nqb > 1 && total_tiles / p.parts > kPaceMinTiles && pace && atoi(pace)) {
-    p.progress = (int*)cvb_ws(ctx, WS_XT_PROGRESS, sizeof(int) * (size_t)p.nqb * p.parts);
-    if (!p.progress) return CVB_ERR_CUDA;
-    CVB_CUDA(ctx, cudaMemsetAsync(p.progress, 0, sizeof(int) * (size_t)p.nqb * p.parts, st));
-  }
+int launch_xt(cvb_ctx* ctx, const TcParams& p, cudaStream_t st) {
   static cvb_once_per_device once;
   if (once.first(ctx->device)) {
     CVB_CUDA(ctx, cudaFuncSetAttribute(tc_xt_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
@@ -1023,41 +831,34 @@ int expand_tiles(cvb_ctx* ctx, const uint8_t* d_rows, const int32_t* d_seg_ptr, 
   return CVB_OK;
 }
 
-template <class M, int K>
+template <int K>
 int launch_tc(cvb_ctx* ctx, const TcParams& p, cudaStream_t st) {
   static cvb_once_per_device once;
-  const size_t smem = smem_bytes<M, K>();
+  const size_t smem = smem_bytes<K>();
   if (once.first(ctx->device)) {
-    CVB_CUDA(ctx, cudaFuncSetAttribute(tc_scan_kernel<M, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CVB_CUDA(ctx, cudaFuncSetAttribute(tc_scan_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   }
-  tc_scan_kernel<M, K><<<p.nqb * p.parts, NUM_THREADS, smem, st>>>(p);
+  tc_scan_kernel<K><<<p.nqb * p.parts, NUM_THREADS, smem, st>>>(p);
   CVB_CHECK_LAUNCH(ctx);
-  if (p.dbg & 16) {
-    static long long h[3][TRACE_TILES][4];
-    CVB_CUDA(ctx, cudaStreamSynchronize(st));
-    CVB_CUDA(ctx, cudaMemcpyFromSymbol(h, g_tc_trace, sizeof(h)));
-    const long long t0 = h[0][0][0];
-    fprintf(stderr, "tile | producer: wait_begin got_slot stored arrived | mma: begin full_ok tempty_ok issued | epilogue: begin tfull_ok done arrived\n");
-    for (int n = 0; n < TRACE_TILES; n++) {
-      fprintf(stderr, "%3d |", n);
-      for (int r = 0; r < 3; r++) {
-        for (int c = 0; c < 4; c++) fprintf(stderr, " %7lld", h[r][n][c] - t0);
-        fprintf(stderr, " |");
-      }
-      fprintf(stderr, "\n");
-    }
-  }
   return CVB_OK;
 }
 
-bool profitable(const cvb_ctx* ctx, int nq, int n_seg, long total_rows, int max_seg_len) {
-  if (max_seg_len >= (1 << kIdxBits)) return false;   // packed (distance, index) keys need < 4 Mi rows per segment
+Formulation choose(const cvb_ctx* ctx, int nq, int n_seg, int64_t total_rows, int max_seg_len, bool filter) {
   const char* e = getenv("COVINS_B200_MATCH_KERNEL");
-  if (e && !strcmp(e, "popc")) return false;
-  if (e && !strcmp(e, "tc")) return n_seg >= 1 && nq >= 1;
+  const bool popc = e && !strcmp(e, "popc"), tc = e && !strcmp(e, "tc");
   const int nqb = (nq + TM - 1) / TM;
-  const int want_parts = ctx->sm_count / nqb > 0 ? ctx->sm_count / nqb : 1;
-  return n_seg >= want_parts && (long)nq * total_rows >= (1L << 26);
+  const int parts = ctx->sm_count / nqb > 0 ? ctx->sm_count / nqb : 1;   // CTAs per query block that fill the GPU
+  const bool big = (int64_t)nq * total_rows >= ((int64_t)1 << 26);
+  // packed (distance, index) keys need < 4 Mi rows per segment
+  if (max_seg_len < (1 << kIdxBits) && (tc ? (n_seg >= 1 && nq >= 1) : (!popc && n_seg >= parts && big))) return {Formulation::kPerSegment, 0};
+  // one very long segment (map-wide k-NN): too few segments to spread over the SMs → about 4 uniform chunks per CTA, each
+  // a multiple of TN and below the key's index range
+  if (!filter && n_seg == 1 && !popc && big && total_rows >= (int64_t)parts * 4 * 1024) {
+    const int64_t n_ps = parts * 4;
+    const int64_t chunk = ((total_rows + n_ps - 1) / n_ps + TN - 1) / TN * TN;
+    return {Formulation::kChunked, std::min(chunk, ((int64_t)1 << kIdxBits) - TN)};
+  }
+  return {Formulation::kScalar, 0};
 }
 
 int launch(cvb_ctx* ctx, TcParams p, int metric, int k, cudaStream_t st) {
@@ -1066,11 +867,7 @@ int launch(cvb_ctx* ctx, TcParams p, int metric, int k, cudaStream_t st) {
   if (parts < 1) parts = 1;
   if (parts > p.n_seg) parts = p.n_seg;
   p.parts = parts;
-  {
-    const char* d = getenv("COVINS_B200_TC_DEBUG");
-    p.dbg = d ? atoi(d) : 0;
-  }
-  if (metric == 0 && !(getenv("COVINS_B200_TC_XT") && !strcmp(getenv("COVINS_B200_TC_XT"), "0"))) {
+  if (metric == 0) {
     if (!p.xt) {
       // no resident tile store for this train set (raw-pointer API): expand it into the workspace first (HBM-bound pre-pass)
       CVB_REQUIRE(ctx, p.h_seg != nullptr, "tensor-core Hamming path needs the host copy of the segment table");
@@ -1086,20 +883,19 @@ int launch(cvb_ctx* ctx, TcParams p, int metric, int k, cudaStream_t st) {
       p.xt = d_xt;
       p.seg_tile = d_tile;
     }
-    const long total_tiles = (long)tiles_of(p.h_seg, p.n_seg, nullptr);
     switch (k) {
-      case 1: return xt::launch_xt<1>(ctx, p, total_tiles, st);
-      case 2: return xt::launch_xt<2>(ctx, p, total_tiles, st);
-      case 3: return xt::launch_xt<3>(ctx, p, total_tiles, st);
-      default: return xt::launch_xt<4>(ctx, p, total_tiles, st);
+      case 1: return xt::launch_xt<1>(ctx, p, st);
+      case 2: return xt::launch_xt<2>(ctx, p, st);
+      case 3: return xt::launch_xt<3>(ctx, p, st);
+      default: return xt::launch_xt<4>(ctx, p, st);
     }
   }
-#define TC_CASE(MM, KK) return launch_tc<MM, KK>(ctx, p, st)
-  if (metric == 0) {
-    switch (k) { case 1: TC_CASE(TcHamming, 1); case 2: TC_CASE(TcHamming, 2); case 3: TC_CASE(TcHamming, 3); default: TC_CASE(TcHamming, 4); }
+  switch (k) {
+    case 1: return launch_tc<1>(ctx, p, st);
+    case 2: return launch_tc<2>(ctx, p, st);
+    case 3: return launch_tc<3>(ctx, p, st);
+    default: return launch_tc<4>(ctx, p, st);
   }
-  switch (k) { case 1: TC_CASE(TcL2, 1); case 2: TC_CASE(TcL2, 2); case 3: TC_CASE(TcL2, 3); default: TC_CASE(TcL2, 4); }
-#undef TC_CASE
 }
 
 }  // namespace cvb_tc

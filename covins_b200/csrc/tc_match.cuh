@@ -1,4 +1,4 @@
-// tc_match.cuh — interface of the tcgen05 (tensor-core) matching kernel, see tc_match.cu
+// tc_match.cuh — interface of the tcgen05 (tensor-core) matching kernels, see tc_match.cu
 #pragma once
 #include <vector>
 
@@ -17,9 +17,6 @@ struct TcParams {
   int nqb, parts;           // filled by launch()
   int32_t* out_idx;
   void* out_dist;
-  const uint8_t* skipA;
-  const uint8_t* skipB;
-  int ithr;
   int filter;
   float thr, ratio;
   int32_t* match_train;
@@ -30,21 +27,26 @@ struct TcParams {
   const uint8_t* xt;
   const int32_t* seg_tile;
   const int32_t* h_seg;
-  int* progress;            // filled by launch(): per (part, query block) tile counter of the pacing scheme, or nullptr
-  int dbg;   // development switches (COVINS_B200_TC_DEBUG): 1 = epilogue skips the selection, 2 = producers skip the expansion
 };
 
 // metric 0 = Hamming (32-byte rows), 1 = L2 on u8 (128-byte rows); OpenCV k-NN rule (the DenseMatcher list rule is
 // order dependent and stays on the scalar kernel)
 int launch(cvb_ctx* ctx, TcParams p, int metric, int k, cudaStream_t st);
 
+// Which formulation a k-NN request (nq >= 1) runs.  The tensor-core kernels are chosen when they fill the GPU: over the
+// request's segments when there are enough of them, or — one very long segment, no fused filter — over uniform chunks of
+// `chunk` rows whose lists the caller merges.  COVINS_B200_MATCH_KERNEL (read at every call): `popc` forces the scalar
+// kernel, `tc` the per-segment tensor-core kernel wherever the packed keys can index the segments.
+struct Formulation {
+  enum Kind { kScalar, kPerSegment, kChunked } kind;
+  int64_t chunk;   // kChunked only
+};
+Formulation choose(const cvb_ctx* ctx, int nq, int n_seg, int64_t total_rows, int max_seg_len, bool filter);
+
 // pre-expanded operand store of the Hamming path: 128-row tiles per segment, tile_bytes() each
 int64_t tiles_of(const int32_t* h_seg, int n_seg, std::vector<int32_t>* seg_tile);   // total tiles; optional prefix [n_seg + 1]
 size_t tile_bytes();
 int expand_tiles(cvb_ctx* ctx, const uint8_t* d_rows, const int32_t* d_seg_ptr, const int32_t* d_seg_tile, int seg_lo, int seg_hi,
                  int tile_lo, int n_tiles, uint8_t* d_xt, cudaStream_t st);
-
-// true when the tensor-core kernel fills the GPU for this shape (enough candidate segments per query block)
-bool profitable(const cvb_ctx* ctx, int nq, int n_seg, long total_rows, int max_seg_len);
 
 }  // namespace cvb_tc

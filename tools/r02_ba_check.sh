@@ -3,7 +3,6 @@ O=gpurun_out; mkdir -p $O
 timeout 900 python -m pytest tests/test_gpu_ba.py -x -q -m gpu > $O/r02_pytest6.log 2>&1; echo "pytest rc=$?" >> $O/r02_pytest6.log
 COVINS_SKIP_CPU_BASELINE=1 timeout 600 python bench.py --steps 10 --warmup 3 > $O/r02_bench3.json 2> $O/r02_bench3.err
 COVINS_B200_NO_CHAIN_STREAM=1 COVINS_SKIP_CPU_BASELINE=1 timeout 600 python bench.py --steps 10 --warmup 3 > $O/r02_bench3_nochain.json 2> $O/r02_bench3_nochain.err
-timeout 200 python tools/tc_trace.py > $O/r02_tc_trace2.txt 2>&1
 tail -3 $O/r02_pytest6.log; python - <<'PY'
 import json
 for f in ("r02_bench3.json", "r02_bench3_nochain.json"):
